@@ -31,7 +31,12 @@ ALGO_GFLOP_PER_UTT_STEP = 202.0
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20,
+                    help="timed updates of the tts / tts_ragged / asr / pretrain workloads (both the resident and the "
+                         "end-to-end pass). Bounded legs use their own counts, each reported in its JSON entry: the "
+                         "tts parity leg times max(3, min(K, 6)) updates, the CPU baselines a fixed 3 (asr) or 8 (tts) "
+                         "updates (--impl reference: max(1, min(K, 10))), and hifigan max(1, K // 10) passes over its "
+                         "512 spectrograms")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--batch", type=int, default=WORKLOAD["batch_per_gpu"])
@@ -51,7 +56,13 @@ def parse():
     ap.add_argument("--profile-step", action="store_true",
                     help="run 2 eager warm-up updates, then ONE eager update between cudaProfilerStart/Stop and exit "
                          "(for `ncu --profile-from-start off`); prints no bench line")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="tts workload: after the timed steps, write what the last timed update returned and a seeded "
+                         "sample of the parameters it updated as DIR/<name>.npy (float32), to compare two builds")
+    args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "b200" or args.workload != "tts" or args.profile_step):
+        ap.error("--dump-outputs is implemented for the timed tts workload of --impl b200")
+    return args
 
 
 # ------------------------------------------------------------------------------------------------ clocks
@@ -204,6 +215,38 @@ def _timed_steps(trainer, batches, steps, warmup, world, dev, read_back):
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         ms = t.item()
     return ms, (w0, w1), last, out
+
+
+DUMP_PARAM_SAMPLE = 1 << 22  # 16 MB of fp32 out of the 144.5 M parameters of the TTS model
+
+
+def dump_sample_index(numel):
+    """The fixed, seeded flat indices of the parameter sample (sorted; drawn with replacement)."""
+    import torch
+    idx = torch.randint(0, numel, (min(DUMP_PARAM_SAMPLE, numel),), generator=torch.Generator().manual_seed(0))
+    return idx.sort().values
+
+
+def dump_outputs(path, trainer, out, rank=0):
+    """What one update computed, for comparing two builds output for output: the per-micro-batch losses and logging
+    statistics train_step returns, and a fixed seeded sample of the updated parameters, drawn from model.named_parameters()
+    concatenated in order (so that it does not depend on the trainer's flat buffer layout). Every rank calls it: under the
+    sharded exchange a rank updates only its own shard of the fp32 masters, so they are gathered first (collective);
+    rank 0 writes."""
+    import numpy as np
+    import torch
+    trainer.consolidate()
+    if rank != 0:
+        return
+    losses, stats = out
+    arrays = {"losses": losses}
+    if stats is not None:
+        arrays["stats"] = stats
+    flat = torch.cat([p.detach().reshape(-1).float() for _, p in trainer.model.named_parameters()])
+    arrays["params_sample"] = flat[dump_sample_index(flat.numel()).to(flat.device)]
+    os.makedirs(path, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), t.detach().float().cpu().numpy())
 
 
 def _peaks():
@@ -823,6 +866,8 @@ def main():
     ms_dev, win_dev, _, out = timed(resident, read_back=False)
     launches_step = None
     ms_e2e, win_e2e, last, out = timed(host, read_back=True)
+    if args.dump_outputs:  # the last timed update of the run (end-to-end pass), before anything else runs
+        dump_outputs(args.dump_outputs, trainer, out, rank)
     loss_val = float(out[0][0].item())
     # kernels launched per step: counted once while the step was traced (graph mode replays the same launches)
     K.LAUNCHES = 0

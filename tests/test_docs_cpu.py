@@ -1,15 +1,12 @@
-"""Documentation integrity: reference citations (file:line) in sources, header and docs resolve against the mounted
-reference tree (skipped on the GPU box, where /root/reference does not exist)."""
+"""Documentation integrity: reference citations (file:line) in sources, header and docs resolve against the line counts
+of the reference files stored in tests/golden/ref_pins.json."""
 import os
 import subprocess
 import sys
 
-import pytest
-
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference"), reason="reference tree not mounted")
 def test_reference_citations_resolve():
     r = subprocess.run([sys.executable, os.path.join(ROOT, "tools", "check_citations.py")], capture_output=True,
                        text=True, timeout=300)

@@ -1,14 +1,17 @@
-"""Pins the oracle restatements against the REFERENCE'S OWN CODE.
+"""Pins the oracle restatements and the plugin's host code against the REFERENCE'S OWN CODE.
 
-Two layers:
-* fixtures `tests/golden/ref_*.npz` were produced by `/root/reference/SpeechT5/speecht5/**` itself (unmodified, loaded by
-  `oracle/ref_loader.py`; generator `tests/golden/make_golden_from_ref.py`): weights, inputs, outputs, the reference
-  criterions' loss terms, gradients, its SequenceGenerator's token ids, its compute_mask_indices draws. The oracle is
-  replayed on the stored weights + inputs and must agree to fp32 round-off (tolerances in each test). These run
-  everywhere (no reference tree needed).
-* when the reference tree is mounted (build container), the fixtures are regenerated in memory and must be identical to
-  the committed ones (stale-fixture guard), and the reference runs at real width / long sequences against the oracle.
+Everything the reference computed is stored under tests/golden/, so these tests run without the reference tree:
+* fixtures `tests/golden/ref_*.npz` (generator `tests/golden/make_golden_from_ref.py`, which runs the reference's
+  `speecht5/**` unmodified through `oracle/ref_loader.py`): weights, inputs, outputs, the reference criterions' loss
+  terms, gradients, its SequenceGenerator's token ids, its compute_mask_indices draws. The oracle is replayed on the
+  stored weights + inputs and must agree to fp32 round-off (tolerances in each test).
+* `tests/golden/ref_pins.{npz,json}` (generator `tests/golden/make_golden_ref_pins.py`): the reference at real width /
+  long sequences on seeded weights (outputs stored as a seeded sample of elements), its pre-training criteria on fixed
+  model outputs, and what its arch functions, add_args, criterion dataclass, reduce_metrics and Dictionary return.
+When the reference tree is available, the fixtures are also regenerated in memory and must equal the committed ones
+(stale-fixture guard).
 """
+import json
 import os
 import sys
 
@@ -20,6 +23,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 GOLD = os.path.join(ROOT, "tests", "golden")
 sys.path.insert(0, GOLD)
 import make_golden_from_ref as mg  # noqa: E402  (constants + case builders; touches the reference only inside cases)
+import make_golden_ref_pins as gp  # noqa: E402  (seeded inputs / weights shared with the generator)
 from oracle import ref_loader as rl  # noqa: E402
 
 needs_ref = pytest.mark.skipif(not rl.available(), reason="reference tree not mounted (GPU box): fixtures only")
@@ -34,6 +38,11 @@ def rel(a, b):
 
 def load(name):
     return dict(np.load(os.path.join(GOLD, name + ".npz")))
+
+
+def pins_json():
+    with open(os.path.join(GOLD, "ref_pins.json"), encoding="utf-8") as fh:
+        return json.load(fh)
 
 
 def state_of(blob, prefix="state/"):
@@ -215,95 +224,73 @@ def test_committed_fixture_is_what_the_reference_produces_now(name):
 
 
 @needs_ref
-@pytest.mark.parametrize("T", [199, 499])
+def test_committed_ref_pins_are_what_the_reference_produces_now():
+    """The same stale-data guard for tests/golden/ref_pins.{json,npz}."""
+    assert json.loads(json.dumps(gp.json_pins())) == pins_json()
+    fresh, stored = gp.array_pins(), load("ref_pins")
+    assert set(fresh) == set(stored)
+    for k in fresh:
+        a, b = np.asarray(fresh[k]), stored[k]
+        if a.dtype.kind in "biu":
+            assert np.array_equal(a, b), k
+        else:
+            np.testing.assert_allclose(a, b, rtol=1e-5, atol=1e-6, err_msg=k)
+
+
+@pytest.mark.parametrize("T", gp.ENCODER_T)
 def test_reference_encoder_at_asr_lengths_matches_oracle(T):
     """VERDICT r1 item 2: `TransformerEncoder.forward` of the reference at T = 199 / 499 (relative positions clipped at
-    +-160, key padding) against the oracle encoder, Base width, 2 layers."""
-    from argparse import Namespace
+    +-160, key padding) against the oracle encoder on the same seeded weights, Base width, 2 layers."""
     from oracle.speecht5_oracle import TransformerEncoder, base_args
-    ns = rl.load()
-    over = dict(encoder_layers=2, dropout=0.0, attention_dropout=0.0, activation_dropout=0.0, encoder_layerdrop=0.0)
-    rargs = rl.reference_args(**over)
-    torch.manual_seed(3)
-    enc_ref = ns.encoder.TransformerEncoder(rargs, rl.RefDictionary(mg.VOCAB), None).eval()
-    oargs = base_args(**over)
-    enc = TransformerEncoder(oargs, mg.VOCAB, None).eval()
-    enc.load_state_dict(enc_ref.state_dict())
-    x = torch.randn(2, T, 768, generator=torch.Generator().manual_seed(1))
-    pad = torch.zeros(2, T, dtype=torch.bool)
-    pad[1, T - 37:] = True
+    pins = load("ref_pins")
+    enc = gp.seeded_fill(TransformerEncoder(base_args(**gp.encoder_over()), mg.VOCAB, None), 3).eval()
+    x, pad = gp.encoder_input(T)
     with torch.no_grad():
-        a = enc_ref(x, pad)
         b = enc(x, pad)
-    assert rel(b["encoder_out"][0], a["encoder_out"][0]) < 1e-5
-    assert rel(b["encoder_out_for_ctc"][0], a["encoder_out_for_ctc"][0]) < 1e-5
+    assert rel(gp.sampled(b["encoder_out"][0], T), pins[f"encoder/{T}/encoder_out"]) < 1e-5
+    assert rel(gp.sampled(b["encoder_out_for_ctc"][0], T + 1), pins[f"encoder/{T}/encoder_out_for_ctc"]) < 1e-5
 
 
-@needs_ref
 def test_reference_conv_feature_extractor_real_width_matches_oracle():
-    """ConvFeatureExtractionModel (speech_encoder_prenet.py:277-374) at the real 512 channels, both modes, 1 s of audio."""
-    from oracle.speecht5_oracle_asr import CONV_FEATURE_LAYERS, ConvFeatureExtractionModel, reference_to_oracle_keys
-    ns = rl.load()
-    x = torch.randn(2, 16000, generator=torch.Generator().manual_seed(1)) * 0.1
+    """ConvFeatureExtractionModel (speech_encoder_prenet.py:277-374) at the real 512 channels, both modes, 1 s of audio,
+    on the same seeded weights."""
+    from oracle.speecht5_oracle_asr import CONV_FEATURE_LAYERS, ConvFeatureExtractionModel
+    pins = load("ref_pins")
+    x = gp.conv_input()
     for mode in ("default", "layer_norm"):
-        torch.manual_seed(5)
-        ref = ns.speech_encoder_prenet.ConvFeatureExtractionModel(CONV_FEATURE_LAYERS, 0.0, mode, False).eval()
-        orc = ConvFeatureExtractionModel(CONV_FEATURE_LAYERS, mode, False).eval()
-        orc.load_state_dict(reference_to_oracle_keys(ref.state_dict()))
+        orc = gp.seeded_fill(ConvFeatureExtractionModel(CONV_FEATURE_LAYERS, mode, False), 5).eval()
         with torch.no_grad():
-            assert rel(orc(x), ref(x)) < 1e-5, mode
+            y = orc(x)
+        assert list(y.shape) == pins[f"conv/{mode}/shape"].tolist(), mode
+        assert rel(gp.sampled(y, 5), pins[f"conv/{mode}/out"]) < 1e-5, mode
 
 
-@needs_ref
 def test_reference_generate_speech_matches_oracle_autoregressive_synthesis():
     """`T5TransformerModel.generate_speech` (models/speecht5.py:1188-1249; its always-on prenet dropout disabled with
-    dprenet_dropout_rate 0) against the oracle's synthesis loop: same number of frames, same mel."""
+    dprenet_dropout_rate 0) against the oracle's synthesis loop on the same seeded weights: same number of frames, same
+    mel."""
     from oracle.speecht5_oracle import T5TransformerModelOracle, base_args
-    over = dict(mg.TINY, conv_feature_layers=mg.TINY_CONV, conv_pos=16, conv_pos_groups=4)
-    torch.manual_seed(21)
-    ref = rl.build_reference_model(rl.reference_args(**over), rl.RefTask(mg.VOCAB, "t2s")).eval()
-    orc = T5TransformerModelOracle(base_args(**mg.TINY)).eval()
-    orc.load_state_dict({k: v for k, v in ref.state_dict().items() if k in orc.state_dict()})
-    g = torch.Generator().manual_seed(2)
-    toks = torch.randint(4, 70, (1, 12), generator=g)
-    spk = torch.randn(1, 512, generator=g)
+    want = load("ref_pins")["generate_speech/mel"]
+    orc = gp.seeded_fill(T5TransformerModelOracle(base_args(**mg.TINY)), 21).eval()
+    toks, spk = gp.speech_input()
     with torch.no_grad():
-        a = ref.generate_speech(source=None, src_tokens=toks, spkembs=spk, threshold=0.5, minlenratio=0.0, maxlenratio=2.0)
         b = orc.generate_speech(src_tokens=toks, spkembs=spk, threshold=0.5, minlenratio=0.0, maxlenratio=2.0)
-    assert a[0].shape == b[0].shape
-    assert rel(b[0], a[0]) < 1e-4
+    assert tuple(b[0].shape) == want.shape
+    assert rel(b[0], want) < 1e-4
 
 
-@needs_ref
 def test_reduce_metrics_logs_the_reference_keys_and_values():
     """SpeechT5Criterion.reduce_metrics (criterions/speecht5_criterion.py:123-436) run by the reference itself and by the
     plugin on the same logging outputs: same meter names, same values."""
-    import importlib
-    ns = rl.load()
-    ref_cls = importlib.import_module("speecht5.criterions.speecht5_criterion").SpeechT5Criterion
     from speecht5_b200.criterions import SpeechT5Criterion
     from speecht5_b200.fairseq_shim import metrics as ours
-    t2s = {"loss": 1.5, "l1_loss": 1.0, "l2_loss": 2.0, "bce_loss": 0.5, "sample_size": 1, "ntokens": 100,
-           "nsentences": 4, "enc_dec_attn_loss": 0.01, "encoder_alpha": 1.0, "decoder_alpha": 1.1}
-    s2t = {"loss": 80.0, "ce_loss": 60.0, "ctc_loss": 100.0, "nll_loss": 55.0, "ntokens": 37, "nsentences": 3,
-           "sample_size": 3, "n_correct": 11, "total": 37, "c_errors": 5, "c_total": 30, "w_errors": 2, "wv_errors": 3,
-           "w_total": 9}
-    text = {"loss": 12.0, "bart_loss": 12.0, "ntokens": 50, "sample_size": 50, "loss_prob_perplexity": 0.3,
-            "code_perplexity": 17.0}
-    hub = {"loss": 9.0, "ntokens": 20, "sample_size": 20, "dec_loss": 1.0, "l1_loss": 0.5, "l2_loss": 0.6, "bce_loss": 0.1,
-           "ngpu": 1, "count_m_0": 12, "correct_m_0": 5, "loss_m_0": 7.0, "enc_dec_attn_loss": 0.02}
-    logs = [{"t2s": t2s, "sample_size": 1, "loss": 1.5}, {"t2s": dict(t2s, loss=2.5), "sample_size": 1, "loss": 2.5},
-            {"s2t": s2t, "sample_size": 1, "loss": 80.0 / 3}, {"text_pretrain": text, "sample_size": 1, "loss": 0.24},
-            {"speech_pretrain": hub, "sample_size": 1, "loss": 0.45}]
-    ns.metrics.logged.clear()
-    ns.metrics.derived.clear()
-    ref_cls.reduce_metrics(logs)
+    want = pins_json()["reduce_metrics"]
     ours.reset()
-    SpeechT5Criterion.reduce_metrics(logs)
-    assert set(ours.scalars) == set(ns.metrics.logged), set(ours.scalars) ^ set(ns.metrics.logged)
-    for k, v in ns.metrics.logged.items():
-        assert abs(float(ours.scalars[k]) - float(v)) < 1e-9, k
-    assert set(ours.derived) == set(ns.metrics.derived)
+    SpeechT5Criterion.reduce_metrics(gp.metric_logs())
+    assert set(ours.scalars) == set(want["logged"]), set(ours.scalars) ^ set(want["logged"])
+    for k, v in want["logged"].items():
+        assert abs(float(ours.scalars[k]) - v) < 1e-9, k
+    assert set(ours.derived) == set(want["derived"])
 
 
 def test_train_step_returns_the_reference_logging_shape():
@@ -368,100 +355,69 @@ def _speech_pretrain_sample():
             "src_lengths": torch.tensor([6, 5, 4]), "task_name": "speech_pretrain"}
 
 
+def text_pretrain_sample(pad):
+    tgt = torch.randint(4, 37, (3, 9), generator=torch.Generator().manual_seed(2))
+    tgt[1, 6:] = pad
+    tgt[2, 3:] = pad
+    return {"net_input": {"src_tokens": None}, "target": tgt, "ntokens": int(tgt.ne(pad).sum()), "task_name": "text_pretrain"}
+
+
+def speech_pretrain_kwargs(dec_weight, nomask, weights):
+    return dict(pred_masked_weight=1.0, pred_nomask_weight=nomask, loss_weights=None if weights is None else list(weights),
+                log_keys=["temp"], hubert_weight=0.7, dec_weight=dec_weight)
+
+
 def _close(a, b, tol=1e-5):
     a, b = float(a), float(b)
     return abs(a - b) <= tol * max(1.0, abs(b))
 
 
-@pytest.mark.parametrize("dec_weight,nomask,weights", [(1.0, 0.0, [10.0]), (0.0, 0.5, [10.0, 0.1]), (0.5, 1.0, [10.0, 0.1, 3.0]),
-                                                       (1.0, 0.0, None)])
+def _assert_criterion_matches(pins, key, stub, got, n_got, log_got):
+    """Loss, sample size, every logging key and the gradients on the stub's outputs against the reference's (stored)."""
+    assert n_got == pins[key + "/sample_size"] and _close(got, pins[key + "/loss"])
+    prefix = key + "/log/"
+    log_want = {k[len(prefix):]: v for k, v in pins.items() if k.startswith(prefix)}
+    assert set(log_got) == set(log_want), (sorted(log_got), sorted(log_want))
+    for k, v in log_want.items():
+        assert _close(log_got[k], v), (k, log_got[k], v)
+    got.backward()
+    for n, q in stub.named_parameters():
+        want = pins.get(f"{key}/grad/{n}")
+        if want is None:
+            assert q.grad is None, n
+        else:
+            assert torch.allclose(gp.sampled(q.grad, 7), torch.from_numpy(want), rtol=1e-5, atol=1e-7), n
+
+
+@pytest.mark.parametrize("dec_weight,nomask,weights", gp.SPEECH_PRETRAIN_CASES)
 def test_speech_pretrain_criterion_equals_the_reference_criterion(dec_weight, nomask, weights):
     """speecht5_b200/criterions/speech_pretrain_criterion.py against the reference's own SpeechPretrainCriterion
     (speech_pretrain_criterion.py:50-190, loaded unmodified): loss, sample size, every logging key and the gradients on
     the model outputs, with / without the decoder branch, the unmasked term and 1 / 2 / 3 configured extra weights."""
-    import importlib
     from speecht5_b200.criterions import SpeechPretrainCriterion
-    rl.load()
-    ref_mod = importlib.import_module("speecht5.criterions.speech_pretrain_criterion")
-    task = rl.RefTask(mg.VOCAB, "pretrain")
-    kw = dict(pred_masked_weight=1.0, pred_nomask_weight=nomask, loss_weights=None if weights is None else list(weights),
-              log_keys=["temp"], hubert_weight=0.7, dec_weight=dec_weight)
-    ref_crit = ref_mod.SpeechPretrainCriterion(task, True, **kw)
-    kw["loss_weights"] = None if weights is None else list(weights)
-    our_crit = SpeechPretrainCriterion(task, True, **kw)
-    ms_ref, ms_our = _PretrainStub(4), _PretrainStub(4)
-    want, n_want, log_want = ref_crit(ms_ref, _speech_pretrain_sample())
+    pins = load("ref_pins")
+    key = f"speech_pretrain/{gp.SPEECH_PRETRAIN_CASES.index((dec_weight, nomask, weights))}"
+    our_crit = SpeechPretrainCriterion(rl.RefTask(mg.VOCAB, "pretrain"), True,
+                                       **speech_pretrain_kwargs(dec_weight, nomask, weights))
+    ms_our = _PretrainStub(4)
     got, n_got, log_got = our_crit(ms_our, _speech_pretrain_sample())
-    assert n_got == n_want and _close(got, want)
-    assert set(log_got) == set(log_want), (sorted(log_got), sorted(log_want))
-    for k in log_want:
-        assert _close(log_got[k], log_want[k]), (k, log_got[k], log_want[k])
-    assert ms_our.calls[0].get("only_hubert", False) == ms_ref.calls[0].get("only_hubert", False) == (dec_weight == 0)
-    want.backward()
-    got.backward()
-    for (n, p), q in zip(ms_ref.named_parameters(), ms_our.parameters()):
-        if p.grad is None:
-            assert q.grad is None, n
-        else:
-            assert torch.allclose(q.grad, p.grad, rtol=1e-5, atol=1e-7), n
+    assert ms_our.calls[0].get("only_hubert", False) == bool(pins[key + "/only_hubert"]) == (dec_weight == 0)
+    _assert_criterion_matches(pins, key, ms_our, got, n_got, log_got)
 
 
-@pytest.mark.parametrize("sentence_avg,weights", [(False, [0.1]), (True, [0.1]), (False, [0.1, 2.0])])
+@pytest.mark.parametrize("sentence_avg,weights", gp.TEXT_PRETRAIN_CASES)
 def test_text_pretrain_criterion_equals_the_reference_criterion(sentence_avg, weights):
     """speecht5_b200/criterions/text_pretrain_criterion.py against the reference's TextPretrainCriterion
     (text_pretrain_criterion.py:36-105): padded targets, both sample-size modes, and the reference's weight-list rule
     when more weights than extra terms are configured (it keeps the tail, :74-75)."""
-    import importlib
     from speecht5_b200.criterions import TextPretrainCriterion
-    rl.load()
-    ref_mod = importlib.import_module("speecht5.criterions.text_pretrain_criterion")
+    pins = load("ref_pins")
+    key = f"text_pretrain/{gp.TEXT_PRETRAIN_CASES.index((sentence_avg, weights))}"
     task = rl.RefTask(mg.VOCAB, "pretrain")
-    pad = task.target_dictionary.pad()
-    tgt = torch.randint(4, 37, (3, 9), generator=torch.Generator().manual_seed(2))
-    tgt[1, 6:] = pad
-    tgt[2, 3:] = pad
-    sample = {"net_input": {"src_tokens": None}, "target": tgt, "ntokens": int(tgt.ne(pad).sum()), "task_name": "text_pretrain"}
-    ms_ref, ms_our = _PretrainStub(6, text=True), _PretrainStub(6, text=True)
-    want, n_want, log_want = ref_mod.TextPretrainCriterion(task, sentence_avg, 0.9, list(weights))(ms_ref, sample)
-    got, n_got, log_got = TextPretrainCriterion(task, sentence_avg, 0.9, list(weights))(ms_our, sample)
-    assert n_got == n_want and _close(got, want)
-    assert set(log_got) == set(log_want), (sorted(log_got), sorted(log_want))
-    for k in log_want:
-        assert _close(log_got[k], log_want[k]), (k, log_got[k], log_want[k])
-    want.backward()
-    got.backward()
-    assert torch.allclose(ms_our.logits.grad, ms_ref.logits.grad, rtol=1e-5, atol=1e-7)
-    assert (ms_ref.pp.grad is None and ms_our.pp.grad is None) or torch.allclose(ms_our.pp.grad, ms_ref.pp.grad)
-
-
-def _reference_dictionary_class():
-    """fairseq/data/dictionary.py of the reference, executed unmodified with its five package imports stubbed (utils,
-    binarizer.safe_readline, data.data_utils, file_io.PathManager, tokenizer.tokenize_line: none of them is reached by
-    load / add_symbol / index / string on an in-memory id list)."""
-    import types
-    path = os.path.join(rl.FAIRSEQ, "data", "dictionary.py")
-    names = ["fairseq", "fairseq.utils", "fairseq.binarizer", "fairseq.data", "fairseq.data.data_utils", "fairseq.file_io",
-             "fairseq.tokenizer"]
-    saved = {n: sys.modules.get(n) for n in names}
-    try:
-        mods = {n: types.ModuleType(n) for n in names}
-        mods["fairseq"].utils = mods["fairseq.utils"]
-        mods["fairseq.utils"].item = lambda t: t.item() if hasattr(t, "item") else t
-        mods["fairseq.binarizer"].safe_readline = lambda f: f.readline()
-        mods["fairseq.data"].data_utils = mods["fairseq.data.data_utils"]
-        mods["fairseq.data.data_utils"].post_process = lambda s, sym: s
-        mods["fairseq.file_io"].PathManager = type("PathManager", (), {"get_local_path": staticmethod(lambda p: p)})
-        mods["fairseq.tokenizer"].tokenize_line = lambda line: line.split()
-        sys.modules.update(mods)
-        ns = {"__name__": "fairseq_dictionary_under_test"}
-        exec(compile(open(path).read(), path, "exec"), ns)
-        return ns["Dictionary"]
-    finally:
-        for n, m in saved.items():
-            if m is None:
-                sys.modules.pop(n, None)
-            else:
-                sys.modules[n] = m
+    ms_our = _PretrainStub(6, text=True)
+    got, n_got, log_got = TextPretrainCriterion(task, sentence_avg, 0.9, list(weights))(
+        ms_our, text_pretrain_sample(task.target_dictionary.pad()))
+    _assert_criterion_matches(pins, key, ms_our, got, n_got, log_got)
 
 
 def test_vocabulary_files_load_like_the_reference_dictionary(tmp_path):
@@ -471,20 +427,20 @@ def test_vocabulary_files_load_like_the_reference_dictionary(tmp_path):
     from speecht5_b200.dictionary import Vocabulary
     from speecht5_b200.tasks import SpeechT5Task
     from speecht5_b200.models import make_args
-    Ref = _reference_dictionary_class()
-    words = ["▁", "e", "t", "a", "o", "n", "'", "<weird token>", "zz"]
+    ref = pins_json()["dictionary"]
+    words = gp.VOCAB_WORDS
     (tmp_path / "dict.txt").write_text("".join(f"{w} {100 - i}\n" for i, w in enumerate(words)), encoding="utf-8")
     (tmp_path / "dict.km.txt").write_text("".join(f"{i} 1\n" for i in range(25)), encoding="utf-8")
-    ref, got = Ref.load(str(tmp_path / "dict.txt")), Vocabulary.load(str(tmp_path / "dict.txt"))
-    assert len(got) == len(ref) == 4 + len(words) and got.symbols == ref.symbols and got.indices == ref.indices
-    assert (got.bos(), got.pad(), got.eos(), got.unk()) == (ref.bos(), ref.pad(), ref.eos(), ref.unk()) == (0, 1, 2, 3)
+    got = Vocabulary.load(str(tmp_path / "dict.txt"))
+    assert len(got) == ref["len"] == 4 + len(words) and got.symbols == ref["symbols"] and got.indices == ref["indices"]
+    assert [got.bos(), got.pad(), got.eos(), got.unk()] == ref["specials"] == [0, 1, 2, 3]
     for w in words + ["missing", "<pad>"]:
-        assert got.index(w) == ref.index(w)
-    assert got.add_symbol("<mask>") == ref.add_symbol("<mask>") and got.add_symbol("e") == ref.add_symbol("e")
-    assert got.count == ref.count and got[999] == ref[999]
-    ids = torch.tensor([[0, 5, 6, 3, 2, 1], [7, 8, 4, 2, 1, 1]])
-    assert got.string(ids, extra_symbols_to_ignore={1}) == ref.string(ids, extra_symbols_to_ignore={1})
-    assert got.string(ids[0], include_eos=True, unk_string="?") == ref.string(ids[0], include_eos=True, unk_string="?")
+        assert got.index(w) == ref["index"][w]
+    assert [got.add_symbol("<mask>"), got.add_symbol("e")] == ref["add_symbol"]
+    assert list(got.count) == ref["count"] and got[999] == ref["item_999"]
+    ids = torch.tensor(gp.VOCAB_IDS)
+    assert got.string(ids, extra_symbols_to_ignore={1}) == ref["string_ignore_pad"]
+    assert got.string(ids[0], include_eos=True, unk_string="?") == ref["string_eos_unk"]
     (tmp_path / "dup.txt").write_text("a 1\na 2\n")
     with pytest.raises(RuntimeError):
         Vocabulary.load(str(tmp_path / "dup.txt"))
@@ -501,46 +457,29 @@ def test_vocabulary_files_load_like_the_reference_dictionary(tmp_path):
     assert model.hubert_layer is not None
 
 
-@needs_ref
-@pytest.mark.parametrize("arch", ["t5_transformer", "t5_transformer_base", "t5_transformer_large", "t5_transformer_base_asr"])
+@pytest.mark.parametrize("arch", gp.ARCHS)
 def test_arch_presets_equal_the_reference_arch_functions(arch):
     """models/speecht5.py:1252-1447: every option both sides know gets the value the reference's OWN arch function
     assigns (run unmodified through oracle/ref_loader.py) -- layer counts, widths, dropouts, extractor mode, final_dim,
     codebook sizes, positional options: what decides whether a reference checkpoint loads and trains the same."""
     from speecht5_b200.models import make_args
-    ref = vars(rl.reference_args(arch=arch))
-    ours = vars(make_args(arch))
+    ref = pins_json()["arch_presets"][arch]
+    ours = gp.plain(vars(make_args(arch)))
     shared = [k for k in ours if k in ref]
     assert len(shared) >= 80
     for k in ("final_dim", "latent_vars", "latent_groups", "latent_temp", "codebook_prob", "logit_temp", "extractor_mode",
               "use_conv_pos", "use_sinc_pos", "untie_final_proj", "label_rates"):
         assert k in shared, k
-    def same(a, b):
-        return tuple(a) == tuple(b) if isinstance(a, (list, tuple)) and isinstance(b, (list, tuple)) else a == b
-    diff = {k: (ours[k], ref[k]) for k in shared if not same(ours[k], ref[k])}
+    diff = {k: (ours[k], ref[k]) for k in shared if ours[k] != ref[k]}
     assert not diff, diff
 
 
-@needs_ref
 def test_criterion_config_defaults_equal_the_reference_dataclass():
     """speecht5_criterion.py:23-30: fairseq builds the criterion from this dataclass, so its defaults decide what a
     recipe that omits a flag trains with. Every field both sides define has the reference's default (sentence_avg is an
     interpolation of optimization.sentence_avg there)."""
-    import dataclasses
-    import importlib
     from speecht5_b200.criterions.speecht5_criterion import SpeechT5CriterionConfig
-    rl.load()
-    ref_cls = importlib.import_module("speecht5.criterions.speecht5_criterion").SpeechT5CriterionConfig
-
-    def defaults(cls):
-        out = {}
-        for f in dataclasses.fields(cls):
-            if f.default is not dataclasses.MISSING:
-                out[f.name] = f.default
-            elif f.default_factory is not dataclasses.MISSING:
-                out[f.name] = f.default_factory()
-        return out
-    ref, ours = defaults(ref_cls), defaults(SpeechT5CriterionConfig)
+    ref, ours = pins_json()["criterion_config_defaults"], gp.plain(gp.dataclass_defaults(SpeechT5CriterionConfig))
     shared = [k for k in ours if k in ref and k != "sentence_avg"]
     assert len(shared) >= 20
     diff = {k: (ours[k], ref[k]) for k in shared
@@ -548,23 +487,15 @@ def test_criterion_config_defaults_equal_the_reference_dataclass():
     assert not diff, diff
 
 
-@needs_ref
 def test_model_command_line_options_cover_the_reference_add_args():
     """models/speecht5.py:117-560 (T5TransformerModel.add_args of the reference, run unmodified): every option it
     defines is defined here with the same value type and choices, so a recipe's command line -- README fine-tuning
     commands pass --freeze-encoder-updates, --mask-prob, --mask-channel-prob, --feature-grad-mult -- parses under this
     plugin; ours adds only the two opt-in builders."""
-    import argparse
     from speecht5_b200.models import T5TransformerModel
-    ns = rl.load()
-
-    def opts(cls):
-        p = argparse.ArgumentParser(allow_abbrev=False)
-        cls.add_args(p)
-        return p, {a.dest: (tuple(a.option_strings), type(a).__name__, getattr(a.type, "__name__", a.type),
-                            tuple(a.choices) if a.choices else None) for a in p._actions if a.dest != "help"}
-    _, ref = opts(ns.T5TransformerModel)
-    parser, ours = opts(T5TransformerModel)
+    ref = pins_json()["model_options"]
+    parser, ours = gp.model_options(T5TransformerModel)
+    ours = gp.plain(ours)
     assert sorted(k for k in ref if k not in ours) == []
     assert sorted(k for k in ours if k not in ref) == ["build_speech_encoder", "build_text_decoder"]
     loose = {"latent_temp", "mask_selection", "mask_channel_selection"}  # (str vs literal_eval / untyped: same strings accepted)
@@ -577,33 +508,18 @@ def test_model_command_line_options_cover_the_reference_add_args():
     assert not hasattr(got, "encoder_layers")  # unset options fall through to the arch function
 
 
-@needs_ref
 def test_task_command_line_options_equal_the_reference_add_args():
     """tasks/speecht5.py:44-213 (SpeechT5Task.add_args; the module itself needs fairseq's data package, so its
     add_argument calls are read from the source text): same flags, value types, defaults, choices and actions here."""
-    import ast
     from speecht5_b200.tasks.speecht5 import SpeechT5Task
-    src = open("/root/reference/SpeechT5/speecht5/tasks/speecht5.py").read()
-    ref = {}
-    for node in ast.walk(ast.parse(src)):
-        if isinstance(node, ast.Call) and isinstance(node.func, ast.Attribute) and node.func.attr == "add_argument":
-            flags = [a.value for a in node.args if isinstance(a, ast.Constant)]
-            kw = {}
-            for k in node.keywords:
-                if k.arg in ("help", "metavar"):
-                    continue
-                try:
-                    kw[k.arg] = ast.literal_eval(k.value)
-                except ValueError:
-                    kw[k.arg] = getattr(k.value, "id", None) or ast.unparse(k.value)
-            ref[flags[-1]] = kw
+    ref = pins_json()["task_options"]
     ours = {}
     for flag, kw in SpeechT5Task._OPTIONS:
         kw = {k: (getattr(v, "__name__", v) if k == "type" else v) for k, v in kw.items() if k not in ("help", "metavar")}
-        ours[flag] = kw
+        ours[flag] = gp.plain(kw)
     assert sorted(k for k in ref if k not in ours) == ["data"]  # (the positional argument, added in add_args itself)
     assert sorted(k for k in ours if k not in ref) == []
-    ref["--t5-task"]["choices"] = SpeechT5Task.TASK_NAME  # (the reference names its list the same way, :40)
+    ref["--t5-task"]["choices"] = gp.plain(SpeechT5Task.TASK_NAME)  # (the reference names its list the same way, :40)
     diff = {k: (ours[k], ref[k]) for k in ours if ours[k] != ref[k]}
     assert not diff, diff
     assert len(ours) >= 35

@@ -13,15 +13,17 @@ import torch.multiprocessing as mp
 sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
 
 
-def _build(dtype):
+def _build(dtype, patch):
+    """`patch`: pytest's monkeypatch in the test process (undone after the test, so later tests see the real kernels),
+    gemm_emulator.Patcher() in a spawned worker."""
     import gemm_emulator
     from helpers import NO_DROPOUT, TINY
     from speecht5_b200.criterions import SpeechT5Criterion
     from speecht5_b200.models import make_args
     from speecht5_b200.ops import RT
     from speecht5_b200.tasks import SpeechT5Task
-    gemm_emulator.install_trainer(gemm_emulator.Patcher())
-    RT.dtype = dtype
+    gemm_emulator.install_trainer(patch)
+    patch.setattr(RT, "dtype", dtype)
     RT.disable_device_seed()
     RT.clear_static()
     RT.invalidate_shadows()
@@ -38,9 +40,9 @@ def _batches():
     return [[synthetic_tts_batch(2, 13, 20, seed=10 * step + r) for r in range(2)] for step in range(2)]
 
 
-def _run_single(dtype, q=None):
+def _run_single(dtype, patch):
     from speecht5_b200.trainer import B200Trainer
-    task, model, crit = _build(dtype)
+    task, model, crit = _build(dtype, patch)
     tr = B200Trainer(model, crit, task, lr=1e-2, use_cuda_graph=False)
     for step in _batches():
         tr.train_step(step)  # two micro-batches per update == two ranks with one each
@@ -50,8 +52,9 @@ def _run_single(dtype, q=None):
 def _worker(rank, world, port, mode, q):
     os.environ.update(MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port))
     dist.init_process_group("gloo", rank=rank, world_size=world)
+    import gemm_emulator
     from speecht5_b200.trainer import B200Trainer
-    task, model, crit = _build(torch.bfloat16)
+    task, model, crit = _build(torch.bfloat16, gemm_emulator.Patcher())
     tr = B200Trainer(model, crit, task, lr=1e-2, use_cuda_graph=False, exchange=mode)
     for step in _batches():
         tr.train_step([step[rank]])
@@ -70,12 +73,12 @@ def _worker(rank, world, port, mode, q):
 
 
 @pytest.mark.parametrize("mode", ["shard", "allreduce"])
-def test_two_rank_exchange_equals_two_micro_batches_on_one_rank(mode):
+def test_two_rank_exchange_equals_two_micro_batches_on_one_rank(mode, monkeypatch):
     """legacy_distributed_data_parallel.py:76-165 + trainer.py:776-826: the mean over ranks of per-rank normalised
     gradients. Both exchanges (reduce-scatter + sharded Adam + all-gather; per-stage all-reduce) give the parameters a
     single process reaches with the two batches as micro-batches; every stage's exchange is launched from its backward
     hook (ADVICE r1: the old hook never fired)."""
-    ref, tr1 = _run_single(torch.bfloat16)
+    ref, tr1 = _run_single(torch.bfloat16, monkeypatch)
     gn1 = tr1.grad_norm()
     ctx = mp.get_context("spawn")
     q = ctx.Queue()
@@ -100,9 +103,9 @@ def test_two_rank_exchange_equals_two_micro_batches_on_one_rank(mode):
         assert (res[0][1][n] == res[1][1][n]).all(), n  # ranks agree bit for bit
 
 
-def test_optimizer_state_round_trip_and_overflow_guard():
+def test_optimizer_state_round_trip_and_overflow_guard(monkeypatch):
     from speecht5_b200.trainer import B200Trainer
-    ref, tr = _run_single(torch.float32)
+    ref, tr = _run_single(torch.float32, monkeypatch)
     sd = tr.state_dict()
     assert set(sd) >= {"state", "param_groups"} and sd["state"][0]["step"] == 2
     assert sd["param_groups"][0]["betas"] == (0.9, 0.98)
@@ -118,7 +121,7 @@ def test_optimizer_state_round_trip_and_overflow_guard():
         tr.check_overflow()
     tr.check_overflow()  # counter was reset
     # round trip into a fresh trainer: same next update
-    task, model, crit = _build(torch.float32)
+    task, model, crit = _build(torch.float32, monkeypatch)
     model.load_state_dict({n: p for n, p in ref.items()})
     tr2 = B200Trainer(model, crit, task, lr=1e-2, use_cuda_graph=False)
     tr2.load_state_dict(sd)
@@ -130,12 +133,12 @@ def test_optimizer_state_round_trip_and_overflow_guard():
         assert torch.allclose(p, a[n], atol=1e-7), n
 
 
-def test_static_shadows_follow_load_state_dict():
+def test_static_shadows_follow_load_state_dict(monkeypatch):
     """ADVICE r1: fairseq builds the trainer first and loads the checkpoint second; the flat bf16 shadow the GEMMs read
     must follow."""
     from speecht5_b200.ops import RT
     from speecht5_b200.trainer import B200Trainer
-    task, model, crit = _build(torch.bfloat16)
+    task, model, crit = _build(torch.bfloat16, monkeypatch)
     tr = B200Trainer(model, crit, task, use_cuda_graph=False)
     w = model.encoder.layers[0].fc1.weight
     new = {k: v.clone() for k, v in model.state_dict().items()}
@@ -146,9 +149,9 @@ def test_static_shadows_follow_load_state_dict():
     assert hi.data_ptr() == tr.fp.shadow[tr.fp.offsets[id(w)]:].data_ptr()  # still the static view, refreshed
 
 
-def test_stage_layout_is_world_divisible_and_ordered():
+def test_stage_layout_is_world_divisible_and_ordered(monkeypatch):
     from speecht5_b200.trainer import FlatParams
-    task, model, crit = _build(torch.bfloat16)
+    task, model, crit = _build(torch.bfloat16, monkeypatch)
     fp = FlatParams(model, world=8, rank=3)
     keys = list(fp.stages)
     assert keys == sorted(keys, key=lambda k: (k[0] != "enc", k[1])) and len(keys) == 4
@@ -212,7 +215,8 @@ def test_packed_device_copies_keep_structure_and_share_one_buffer():
 
 
 # ------------------------------------------------------------------------- joint pre-training update on two ranks
-def _pretrain_build():
+def _pretrain_build(patch):
+    """`patch` as in _build."""
     import gemm_emulator
     from helpers import NO_DROPOUT, TINY
     from speecht5_b200 import frontend
@@ -220,11 +224,10 @@ def _pretrain_build():
     from speecht5_b200.models import make_args
     from speecht5_b200.ops import RT
     from speecht5_b200.tasks import SpeechT5Task
-    p = gemm_emulator.Patcher()
-    gemm_emulator.install_autograd(p)
-    gemm_emulator.install_trainer(p)
-    frontend.ConvFeatureExtractor.forward = lambda self, wave: self._layers(wave)  # (no CUDA guard: emulated kernels)
-    RT.dtype = torch.bfloat16
+    gemm_emulator.install_autograd(patch)
+    gemm_emulator.install_trainer(patch)
+    patch.setattr(frontend.ConvFeatureExtractor, "forward", lambda self, wave: self._layers(wave))  # (no CUDA guard)
+    patch.setattr(RT, "dtype", torch.bfloat16)
     RT.disable_device_seed()
     RT.clear_static()
     RT.invalidate_shadows()
@@ -252,8 +255,9 @@ def _pretrain_batches(r):
 def _pretrain_worker(rank, world, port, mode, q):
     os.environ.update(MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port))
     dist.init_process_group("gloo", rank=rank, world_size=world)
+    import gemm_emulator
     from speecht5_b200.trainer import B200Trainer
-    task, model, crit = _pretrain_build()
+    task, model, crit = _pretrain_build(gemm_emulator.Patcher())
     tr = B200Trainer(model, crit, task, lr=1e-2, use_cuda_graph=False, exchange=mode)
     for _ in range(2):
         tr.train_step(_pretrain_batches(rank))
@@ -264,14 +268,14 @@ def _pretrain_worker(rank, world, port, mode, q):
 
 
 @pytest.mark.parametrize("mode", ["shard", "allreduce"])
-def test_two_rank_joint_pretraining_update_equals_four_micro_batches_on_one_rank(mode):
+def test_two_rank_joint_pretraining_update_equals_four_micro_batches_on_one_rank(mode, monkeypatch):
     """The pre-training recipe trains with `--find-unused-parameters` (README): the text micro-batch -- the LAST one of an
     update -- never touches the waveform front end, the masked-prediction head or the speech decoder pre/post-net, and
     the speech one never touches the text pre/post-nets. Stages whose backward hook does not fire on the last
     micro-batch are exchanged at the end of the update: two ranks with (speech_r, text_r) each reach the parameters one
     process reaches with the four micro-batches."""
     from speecht5_b200.trainer import B200Trainer
-    task, model, crit = _pretrain_build()
+    task, model, crit = _pretrain_build(monkeypatch)
     tr = B200Trainer(model, crit, task, lr=1e-2, use_cuda_graph=False)
     for _ in range(2):
         tr.train_step(_pretrain_batches(0) + _pretrain_batches(1))
@@ -297,5 +301,51 @@ def test_two_rank_joint_pretraining_update_equals_four_micro_batches_on_one_rank
         assert (res[0][1][n] == res[1][1][n]).all(), n
     moved = [n for n in ("speech_encoder_prenet.feature_extractor.conv_layers.0.0.weight", "hubert_layer.label_embs_concat",
                          "text_encoder_prenet.encoder_prenet.0.weight", "speech_decoder_postnet.feat_out.weight")
-             if not torch.equal(ref[n], dict(_pretrain_build()[1].named_parameters())[n].detach())]
+             if not torch.equal(ref[n], dict(_pretrain_build(monkeypatch)[1].named_parameters())[n].detach())]
     assert len(moved) == 4, moved
+
+
+# ------------------------------------------------------------------------- bench.py --dump-outputs on two ranks
+def _dump_worker(rank, world, port, path, q):
+    os.environ.update(MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port))
+    dist.init_process_group("gloo", rank=rank, world_size=world)
+    import bench
+    import gemm_emulator
+    from speecht5_b200.trainer import B200Trainer
+    task, model, crit = _build(torch.bfloat16, gemm_emulator.Patcher())
+    tr = B200Trainer(model, crit, task, lr=1e-2, use_cuda_graph=False, exchange="shard")
+    for step in _batches():
+        out = tr.train_step([step[rank]])
+    bench.dump_outputs(path, tr, out, rank)
+    q.put(rank)
+    dist.barrier()
+    dist.destroy_process_group()
+
+
+def test_bench_dump_of_a_sharded_update_holds_the_updated_parameters(monkeypatch, tmp_path):
+    """bench.py --dump-outputs under --gpus 2 with the sharded exchange, where each rank runs Adam only on its own shard
+    of the fp32 masters: the parameter sample rank 0 writes is the model one process reaches with both batches as
+    micro-batches, not rank 0's stale copy of the other rank's shards."""
+    import numpy as np
+    import bench
+    ref, _ = _run_single(torch.bfloat16, monkeypatch)
+    init = _build(torch.bfloat16, monkeypatch)[1]
+    want = torch.cat([p.reshape(-1).float() for p in ref.values()])
+    before = torch.cat([p.detach().reshape(-1).float() for p in init.parameters()])
+    idx = bench.dump_sample_index(want.numel())
+    ctx = mp.get_context("spawn")
+    q = ctx.Queue()
+    port = 29311 + os.getpid() % 300
+    path = str(tmp_path / "dump")
+    procs = [ctx.Process(target=_dump_worker, args=(r, 2, port, path, q)) for r in range(2)]
+    for p in procs:
+        p.start()
+    res = sorted([q.get(timeout=300) for _ in range(2)])
+    for p in procs:
+        p.join(timeout=60)
+    assert res == [0, 1]
+    assert sorted(os.listdir(path)) == ["losses.npy", "params_sample.npy", "stats.npy"]
+    got = torch.from_numpy(np.load(os.path.join(path, "params_sample.npy")))
+    assert got.shape == idx.shape
+    assert (got != before[idx]).float().mean().item() > 0.9
+    assert ((got - want[idx]).norm() / want[idx].norm()).item() < 2e-3

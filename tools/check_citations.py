@@ -1,40 +1,31 @@
 """Checks that every reference citation of the form `<path>.py:<line>[-<line>]` in the repo's sources and docs names a
-file that exists under /root/reference (SpeechT5 tree first, sibling trees second) and a line range inside it. Runs
-only where the reference is mounted (this container); prints the broken ones and exits 1 if any.
+reference file (SpeechT5 tree first, sibling trees second) and a line range inside it. The line counts of the cited
+reference files are stored in tests/golden/ref_pins.json (`reference_line_counts`, written from the reference by
+tests/golden/make_golden_ref_pins.py, which must be re-run when a citation names a file not listed there). Prints the
+broken ones and exits 1 if any.
 usage: python tools/check_citations.py [-v]"""
 import glob
+import json
 import os
 import re
 import sys
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference"
+PINS = os.path.join(ROOT, "tests", "golden", "ref_pins.json")
 ALIAS = {"legacy_ddp.py": "fairseq/distributed/legacy_distributed_data_parallel.py"}  # SURVEY.md:15 shorthand
 PAT = re.compile(r"([A-Za-z0-9_./-]+\.py):(\d+)(?:-(\d+))?")
+UNCHECKED = ("SURVEY.md", "PAPERS.md", "SNIPPETS.md", "BASELINE.md", "VERDICT.md", "ADVICE.md")
 
 
-def index():
-    by_tail = {}
-    for p in glob.glob(REF + "/**/*.py", recursive=True):
-        rel = p[len(REF) + 1:]
-        parts = rel.split("/")
-        for i in range(len(parts)):
-            by_tail.setdefault("/".join(parts[i:]), []).append(p)
-    return by_tail
-
-
-def main():
-    verbose = "-v" in sys.argv
-    if not os.path.isdir(REF):
-        print("reference not mounted; nothing checked")
-        return 0
-    by_tail = index()
+def citations(root=ROOT):
+    """(reference path, first line, last line, citing file, its line number, citation text) of every citation in the
+    sources and docs that does not name a file of this repository."""
     files = [p for pat in ("*.md", "include/*.h", "oracle/*.py", "speecht5_b200/**/*.py", "speecht5_b200/csrc/*",
                            "tests/**/*.py", "bench.py", "__graft_entry__.py")
-             for p in glob.glob(os.path.join(ROOT, pat), recursive=True)]
-    lens, bad, n = {}, [], 0
+             for p in glob.glob(os.path.join(root, pat), recursive=True)]
+    out = []
     for f in sorted(set(files)):
-        if os.path.basename(f) in ("SURVEY.md", "PAPERS.md", "SNIPPETS.md", "BASELINE.md", "VERDICT.md", "ADVICE.md"):
+        if os.path.basename(f) in UNCHECKED:
             continue
         for ln, line in enumerate(open(f, errors="ignore"), 1):
             for m in PAT.finditer(line):
@@ -42,28 +33,41 @@ def main():
                 if "..." in path:
                     continue
                 path = path.lstrip("./")
-                if path.startswith("root/reference/"):
-                    path = path[len("root/reference/"):]
+                if path.split("/", 2)[:2] == ["root", "reference"]:  # an absolute path into the reference checkout
+                    path = path.split("/", 2)[2]
                 path = ALIAS.get(path, path)
-                if os.path.exists(os.path.join(ROOT, path)):  # a citation of this repo's own file
+                if os.path.exists(os.path.join(root, path)):  # a citation of this repo's own file
                     continue
-                cands = by_tail.get(path)
-                if not cands:
-                    bad.append((f, ln, m.group(0), "no such reference file"))
-                    continue
-                n += 1
-                cands = sorted(cands, key=lambda p: (0 if "/SpeechT5/" in p else 1, len(p)))
-                ok = False
-                for c in cands:
-                    if c not in lens:
-                        lens[c] = sum(1 for _ in open(c, errors="ignore"))
-                    if a <= b <= lens[c]:
-                        ok = True
-                        break
-                if not ok:
-                    bad.append((f, ln, m.group(0), f"line range outside the file ({lens[cands[0]]} lines)"))
-                elif verbose:
-                    print("ok", m.group(0))
+                out.append((path, a, b, f, ln, m.group(0)))
+    return out
+
+
+def index(paths):
+    by_tail = {}
+    for rel in paths:
+        parts = rel.split("/")
+        for i in range(len(parts)):
+            by_tail.setdefault("/".join(parts[i:]), []).append(rel)
+    return by_tail
+
+
+def main():
+    verbose = "-v" in sys.argv
+    with open(PINS, encoding="utf-8") as fh:
+        lens = json.load(fh)["reference_line_counts"]
+    by_tail = index(lens)
+    bad, n = [], 0
+    for path, a, b, f, ln, cite in citations():
+        cands = by_tail.get(path)
+        if not cands:
+            bad.append((f, ln, cite, "no such reference file"))
+            continue
+        n += 1
+        cands = sorted(cands, key=lambda p: (0 if p.startswith("SpeechT5/") else 1, len(p)))
+        if not any(a <= b <= lens[c] for c in cands):
+            bad.append((f, ln, cite, f"line range outside the file ({lens[cands[0]]} lines)"))
+        elif verbose:
+            print("ok", cite)
     for f, ln, cite, why in bad:
         print(f"{f[len(ROOT) + 1:]}:{ln}: {cite}: {why}")
     print(f"{n} citations checked, {len(bad)} broken")
