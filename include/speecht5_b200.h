@@ -308,6 +308,36 @@ int st5_guided_attn_bwd(float* const* datt, int32_t n_layers, int32_t B, int32_t
                         int32_t T_in, int64_t p_ld, const int64_t* ilens, const int64_t* olens, int32_t r, float sigma,
                         float alpha, const float* gsum, const float* g, int32_t zero_rest, void* stream);
 
+/* ------------------------------------------------------------------------------------------------- beam search
+ * Joint CTC/attention beam search (speecht5/sequence_generator.py:273-284, :370-418). All values fp32; the sentinel is
+ * the reference's finite logzero = -1e10. x: CTC log-probabilities, element (b, t, v) at b*ld_b + t*ld_t + v
+ * (ld_t >= V); t_valid [B] int64: valid frames T_b of each utterance (rows t >= T_b are never read). T <= 1500,
+ * K <= 256; outside these limits the call fails (code -2) without a launch.
+ *
+ * st5_ctc_prefix_init replaces CTCPrefixScore.initial_state (espnet ctc_prefix_score.py, numpy on the host): r [B, T, 2]
+ * with r[b, t, 0] = logzero and r[b, t, 1] = sum_{tau <= t} x[b, tau, blank] for t < T_b (logzero beyond). */
+int st5_ctc_prefix_init(const float* x, int64_t ld_b, int64_t ld_t, const int64_t* t_valid, float* r, int32_t B,
+                        int32_t T, int32_t V, int32_t blank, void* stream);
+/* st5_ctc_prefix_score replaces the per-hypothesis CTCPrefixScore.__call__ loop of sequence_generator.py:379-391 (one
+ * host call per hypothesis, each looping over every frame): H hypotheses x K candidate labels in one launch, a CTA per
+ * hypothesis, a thread per candidate. Per hypothesis h: utt[h] (its utterance), r_prev [H, T, 2] (its state), last[h]
+ * (its last label), out_len[h] (prefix length without the leading eos); candidates cs [H, K] int64. Writes
+ * log_psi [H, K] and the candidate states r [H, T, 2, K] (frame-major, candidates innermost). Semantics of the
+ * reference scorer: phi = r_prev_b where the candidate repeats the last label; the recursion starts at frame
+ * max(out_len, 1); an eos candidate gets logaddexp(r_prev_n, r_prev_b) at frame T_b - 1, a blank candidate logzero;
+ * out_len >= T_b leaves the recursion empty; rows the reference leaves uninitialised are logzero. */
+int st5_ctc_prefix_score(const float* x, int64_t ld_b, int64_t ld_t, const int64_t* utt, const float* r_prev,
+                         const int64_t* last, const int64_t* out_len, const int64_t* cs, const int64_t* t_valid,
+                         float* log_psi, float* r, int32_t H, int32_t T, int32_t K, int32_t V, int32_t blank,
+                         int32_t eos, void* stream);
+/* st5_beam_gather_rows replaces the per-layer index_select of the decoder's incremental state on a beam reorder
+ * (sequence_generator.py:358, reorder_incremental_state): for every layer l < n_layers (<= 32) and hypothesis h < H,
+ * copies the first n_rows * row_bytes bytes of src[l] + parent[h] * src_bs to dst[l] + h * dst_bs. src / dst: host
+ * arrays of device pointers (two distinct buffer sets: no in-place reorder). row_bytes, src_bs, dst_bs and every
+ * pointer 16-byte aligned. Only the rows already written are copied, not the whole max_len span. */
+int st5_beam_gather_rows(const void* const* src, void* const* dst, const int64_t* parent, int32_t n_layers, int32_t H,
+                         int32_t n_rows, int64_t row_bytes, int64_t src_bs, int64_t dst_bs, void* stream);
+
 /* ------------------------------------------------------------------------------------------------- optimizer
  * Replaces fairseq/optim/adam.py + fp16_optimizer.py:106-218 on a flat fp32 parameter buffer: one pass applies the
  * gradient scale (grad_mul x clip coefficient max_norm / (norm + 1e-6) capped at 1: fairseq/utils.py clip_grad_norm_,

@@ -100,6 +100,10 @@ _PROTOS = {
                                       _vp]),
     "st5_guided_attn_bwd": (C.c_int, [_vp, _i32, _i32, _i32, _i32, _i32, _i32, _i64, _vp, _vp, _i32, _f, _f, _vp, _vp,
                                       _i32, _vp]),
+    "st5_ctc_prefix_init": (C.c_int, [_vp, _i64, _i64, _vp, _vp, _i32, _i32, _i32, _i32, _vp]),
+    "st5_ctc_prefix_score": (C.c_int, [_vp, _i64, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i32, _i32, _i32, _i32,
+                                       _i32, _i32, _vp]),
+    "st5_beam_gather_rows": (C.c_int, [_vp, _vp, _vp, _i32, _i32, _i32, _i64, _i64, _i64, _vp]),
     "st5_sumsq": (C.c_int, [_vp, _i64, _vp, _vp]),
     "st5_adam_step": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _i64, _f, _f, _f, _f, _f, _i64, _vp, _f, _f, _vp, _vp, _vp]),
 }

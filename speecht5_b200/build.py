@@ -11,7 +11,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "lib", "libspeecht5_b200.so")
 SOURCES = ["api.cu", "gemm.cu", "elementwise.cu", "norm.cu", "layernorm.cu", "attention.cu", "attention_tc.cu", "attention_fused.cu", "attention_fused_bwd.cu", "attention_flash.cu",
-           "optim.cu", "conv_frontend.cu", "ctc.cu", "criterion.cu"]
+           "optim.cu", "conv_frontend.cu", "ctc.cu", "ctc_prefix.cu", "criterion.cu"]
 HEADERS = ["ptx.cuh", "gemm.cuh", "kernels.cuh", "tma_map.cuh", "vec8.cuh", os.path.join("..", "..", "include", "speecht5_b200.h")]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",

@@ -233,6 +233,26 @@ int st5_ctc_loss(const float* logits, int64_t ld_t, int64_t ld_b, const int64_t*
                    "st5_ctc_loss");
 }
 
+int st5_ctc_prefix_init(const float* x, int64_t ld_b, int64_t ld_t, const int64_t* t_valid, float* r, int32_t B,
+                        int32_t T, int32_t V, int32_t blank, void* stream) {
+  return set_error(ctc_prefix_init_launch(x, ld_b, ld_t, t_valid, r, B, T, V, blank, (cudaStream_t)stream),
+                   "st5_ctc_prefix_init");
+}
+int st5_ctc_prefix_score(const float* x, int64_t ld_b, int64_t ld_t, const int64_t* utt, const float* r_prev,
+                         const int64_t* last, const int64_t* out_len, const int64_t* cs, const int64_t* t_valid,
+                         float* log_psi, float* r, int32_t H, int32_t T, int32_t K, int32_t V, int32_t blank,
+                         int32_t eos, void* stream) {
+  return set_error(ctc_prefix_score_launch(x, ld_b, ld_t, utt, r_prev, last, out_len, cs, t_valid, log_psi, r, H, T, K,
+                                           V, blank, eos, (cudaStream_t)stream),
+                   "st5_ctc_prefix_score");
+}
+int st5_beam_gather_rows(const void* const* src, void* const* dst, const int64_t* parent, int32_t n_layers, int32_t H,
+                         int32_t n_rows, int64_t row_bytes, int64_t src_bs, int64_t dst_bs, void* stream) {
+  return set_error(beam_gather_rows_launch(src, dst, parent, n_layers, H, n_rows, row_bytes, src_bs, dst_bs,
+                                           (cudaStream_t)stream),
+                   "st5_beam_gather_rows");
+}
+
 int st5_sumsq(const float* x, int64_t n, float* out, void* stream) {
   return set_error(sumsq_launch(x, n, out, (cudaStream_t)stream), "st5_sumsq");
 }

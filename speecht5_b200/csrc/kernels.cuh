@@ -188,6 +188,14 @@ int ctc_loss_launch(const float* logits, int64_t ld_t, int64_t ld_b, const int64
                     const int64_t* input_lengths, const int64_t* target_lengths, float* nll, float* grad, float* ws,
                     int32_t T, int32_t B, int32_t V, int32_t S_max, int32_t blank, int32_t zero_infinity,
                     cudaStream_t s);
+int ctc_prefix_init_launch(const float* x, int64_t ld_b, int64_t ld_t, const int64_t* t_valid, float* r, int32_t B,
+                           int32_t T, int32_t V, int32_t blank, cudaStream_t s);
+int ctc_prefix_score_launch(const float* x, int64_t ld_b, int64_t ld_t, const int64_t* utt, const float* r_prev,
+                            const int64_t* last, const int64_t* out_len, const int64_t* cs, const int64_t* t_valid,
+                            float* log_psi, float* r_out, int32_t H, int32_t T, int32_t K, int32_t V, int32_t blank,
+                            int32_t eos, cudaStream_t s);
+int beam_gather_rows_launch(const void* const* src, void* const* dst, const int64_t* parent, int32_t L, int32_t H,
+                            int32_t n_rows, int64_t row_bytes, int64_t src_bs, int64_t dst_bs, cudaStream_t s);
 int sumsq_launch(const float* x, int64_t n, float* out, cudaStream_t s);
 int adam_launch(float* p, const float* g, float* m, float* v, void* p_bf16, int64_t n, float lr, float beta1,
                 float beta2, float eps, float weight_decay, int64_t step, const float* grad_norm_sq, float max_norm,

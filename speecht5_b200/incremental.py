@@ -53,6 +53,25 @@ class DecoderCache:
         if self.enc_pad is not None:
             self.enc_pad = self.enc_pad.index_select(0, new_order)
 
+    def gather_rows(self, parent, keep=None):
+        """Beam reorder of the self-attention keys / values: hypothesis h continues parent[h] (int64 [H'] on the device).
+        One st5_beam_gather_rows launch copies the rows written so far (the first `t`) of every layer into a second
+        buffer set, which then becomes the cache (ping-pong: the previous one is reused by the next reorder). `keep`
+        (rows of the hypotheses still decoding, when sentences finished) compacts the cross-attention keys / values and
+        the padding mask; otherwise they stay as they are -- a hypothesis never changes utterance."""
+        from . import kernels as K
+        spare = getattr(self, "_spare", None)
+        if spare is None or spare[0].shape[0] < parent.numel():
+            spare = [torch.empty_like(c) for c in self.self_kv]
+        dst = [s[: parent.numel()] for s in spare]
+        K.beam_gather_rows(self.self_kv, dst, parent, self.t)
+        self._spare = [c if c._base is None else c._base for c in self.self_kv]
+        self.self_kv = dst
+        if keep is not None:
+            self.cross = [c.index_select(0, keep) for c in self.cross]
+            if self.enc_pad is not None:
+                self.enc_pad = self.enc_pad.index_select(0, keep)
+
 
 @torch.no_grad()
 def decoder_step(decoder, x_new, cache, need_head_weights=False, t_dev=None, span=None, self_pad=None):

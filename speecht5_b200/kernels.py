@@ -345,6 +345,59 @@ def ctc_loss(logits, targets, tgt_offsets, input_lengths, target_lengths, nll, g
     _count(3 if grad is not None else 2)
 
 
+def ctc_prefix_init(x, t_valid, r, blank):
+    """x [B, T, V] fp32 CTC log-probabilities (inner stride 1), t_valid [B] int64 -> r [B, T, 2] fp32 (st5_ctc_prefix_init)."""
+    _require_cuda(x, t_valid, r)
+    assert x.dtype == torch.float32 and x.stride(2) == 1 and t_valid.dtype == torch.int64 and t_valid.is_contiguous()
+    B, T, V = x.shape
+    assert r.shape == (B, T, 2) and r.dtype == torch.float32 and r.is_contiguous()
+    lib = _lib.load()
+    _lib.check(lib.st5_ctc_prefix_init(_ptr(x), x.stride(0), x.stride(1), _ptr(t_valid), _ptr(r), B, T, V, blank,
+                                       _stream()), "st5_ctc_prefix_init")
+    _count(1)
+
+
+def ctc_prefix_score(x, t_valid, utt, r_prev, last, out_len, cs, log_psi, r, blank, eos):
+    """Candidate scores log_psi [H, K] and states r [H, T, 2, K] of H hypotheses x K candidate labels cs [H, K]
+    (st5_ctc_prefix_score). x [B, T, V] fp32; utt / last / out_len [H] int64; r_prev [H, T, 2] fp32."""
+    _require_cuda(x, t_valid, utt, r_prev, last, out_len, cs, log_psi, r)
+    assert x.dtype == torch.float32 and x.stride(2) == 1
+    for t in (t_valid, utt, last, out_len, cs):
+        assert t.dtype == torch.int64 and t.is_contiguous()
+    B, T, V = x.shape
+    H, K = cs.shape
+    assert r_prev.shape == (H, T, 2) and r_prev.dtype == torch.float32 and r_prev.is_contiguous()
+    assert log_psi.shape == (H, K) and log_psi.dtype == torch.float32 and log_psi.is_contiguous()
+    assert r.shape == (H, T, 2, K) and r.dtype == torch.float32 and r.is_contiguous()
+    lib = _lib.load()
+    _lib.check(lib.st5_ctc_prefix_score(_ptr(x), x.stride(0), x.stride(1), _ptr(utt), _ptr(r_prev), _ptr(last),
+                                        _ptr(out_len), _ptr(cs), _ptr(t_valid), _ptr(log_psi), _ptr(r), H, T, K, V, blank,
+                                        eos, _stream()), "st5_ctc_prefix_score")
+    _count(1)
+
+
+def beam_gather_rows(src, dst, parent, n_rows):
+    """dst[l][h, :n_rows] = src[l][parent[h], :n_rows] for every layer l (st5_beam_gather_rows): src / dst lists of
+    [*, max_len, W] tensors with contiguous rows, two distinct buffer sets; parent [H] int64 on the device."""
+    _require_cuda(parent, *src, *dst)
+    assert len(src) == len(dst) and parent.dtype == torch.int64 and parent.is_contiguous()
+    H = parent.numel()
+    s0, d0 = src[0], dst[0]
+    row_bytes = s0.stride(1) * s0.element_size()
+    assert s0.stride(2) == 1 and s0.stride(1) == s0.shape[2] and d0.shape[0] >= H
+    for s, d in zip(src, dst):
+        assert s.stride() == s0.stride() and d.stride() == d0.stride() and s.dtype == d.dtype == s0.dtype
+        assert d.stride(1) == s.stride(1) and d.data_ptr() != s.data_ptr()
+    n = len(src)
+    lib = _lib.load()
+    sp = (C.c_void_p * n)(*[s.data_ptr() for s in src])
+    dp = (C.c_void_p * n)(*[d.data_ptr() for d in dst])
+    _lib.check(lib.st5_beam_gather_rows(sp, dp, _ptr(parent), n, H, int(n_rows), row_bytes,
+                                        s0.stride(0) * s0.element_size(), d0.stride(0) * d0.element_size(), _stream()),
+               "st5_beam_gather_rows")
+    _count(1)
+
+
 def tts_loss_ws_floats(B, L):
     return int(_lib.load().st5_tts_loss_ws_floats(B, L))
 

@@ -494,6 +494,22 @@ class T5TransformerModel(FairseqEncoderDecoderModel):
             return hyp, [pos_scores[b, : len(h)].clone() for b, h in enumerate(hyp)]
         return hyp
 
+    @torch.no_grad()
+    def generate_text_beam(self, source, padding_mask=None, beam_size=5, ctc_weight=0.0, max_len_a=0.0, max_len_b=200,
+                           min_len=1, normalize_scores=True, len_penalty=1.0, unk_penalty=0.0, temperature=1.0, pad=1,
+                           eos=2, unk=3, blank=0, mask_idx=None, mask_idxs=None, use_cache=False):
+        """Beam search with optional joint CTC/attention scoring, as `generate.py --beam N --ctc-weight W` runs it
+        (speecht5/sequence_generator.py:207-655; speecht5_b200/beam.py states the two deliberate deviations: per-utterance
+        CTC posteriors at batch > 1, and a defined state for a selected token outside the CTC candidates). Returns, per
+        sentence, min(beam_size, V - 1) hypotheses {"tokens", "score", "positional_scores", "alignment", "attention"}
+        sorted by score. use_cache: False (prefix recomputation), True (key/value cache, rows reordered by
+        st5_beam_gather_rows)."""
+        from ..beam import beam_search
+        return beam_search(self, source, padding_mask, beam_size=beam_size, ctc_weight=ctc_weight, max_len_a=max_len_a,
+                           max_len_b=max_len_b, min_len=min_len, normalize_scores=normalize_scores,
+                           len_penalty=len_penalty, unk_penalty=unk_penalty, temperature=temperature, pad=pad, eos=eos,
+                           unk=unk, blank=blank, mask_idx=mask_idx, mask_idxs=mask_idxs, use_cache=bool(use_cache))
+
     def forward_text_encoder(self, src_tokens):
         encoder_input, encoder_padding_mask = self.text_encoder_prenet(src_tokens)
         return self.encoder(encoder_input, encoder_padding_mask)

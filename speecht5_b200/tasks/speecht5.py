@@ -99,7 +99,9 @@ class SpeechT5Task(LegacyFairseqTask):
         return None
 
     def build_generator(self, models, args, seq_gen_cls=None, extra_gen_cls_kwargs=None):
-        """tasks/speecht5.py:599-613 for beam size 1 (the reference hands its SequenceGenerator the task's ctc_weight)."""
+        """tasks/speecht5.py:599-613 (the reference hands its SequenceGenerator the task's ctc_weight). Without
+        `seq_gen_cls` the generator is GreedyGenerator (beam 1 without CTC scoring; anything else raises); fairseq's
+        `seq_gen_cls` is honoured: seq_gen_cls=BeamSearchGenerator builds the beam search with the same keywords."""
         from ..generator import GreedyGenerator
         kw = dict(beam_size=getattr(args, "beam", 1), max_len_a=getattr(args, "max_len_a", 0),
                   max_len_b=getattr(args, "max_len_b", 200), min_len=getattr(args, "min_len", 1),
@@ -108,7 +110,7 @@ class SpeechT5Task(LegacyFairseqTask):
                   ctc_weight=getattr(self.args, "ctc_weight", 0.0), blank=getattr(self, "blank_symbol_idx", None),
                   mask_idx=getattr(self, "mask_idx", None))
         kw.update(extra_gen_cls_kwargs or {})
-        return GreedyGenerator(models, self.target_dictionary, **kw)
+        return (seq_gen_cls or GreedyGenerator)(models, self.target_dictionary, **kw)
 
     def inference_step(self, generator, models, sample, prefix_tokens=None, constraints=None):
         with torch.no_grad():  # fairseq/tasks/fairseq_task.py inference_step
